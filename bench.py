@@ -29,6 +29,9 @@ The narrow phase is NOT in the step (outside the hot path, SURVEY.md 8f #1); its
                (N = 1 is the baseline of the curve).
   cpu_baseline the CPU oracle (C++ restatement of the reference path, colour-parallel, all host cores) on the same snapshot.
   --impl reference   times only that CPU arm (the reference itself is Rust and cannot be built in this image).
+  --dump-outputs DIR the arrays the last timed step returned (`value`'s arm, or the CPU arm with --impl reference): bodies, impulses, joint
+                     forces, the count of new pairs (and their columns when there are any), persistent order, as DIR/<name>.npy, so that
+                     two builds can be compared output for output.
 """
 from __future__ import annotations
 
@@ -139,6 +142,44 @@ def build_snapshot(scene_name: str, settle: int, ctx=None):
     return sc, w.params, w.bodies, man, aabbs, w.joints
 
 
+DUMP_BUDGET = 60 << 20     # bytes of array data per --dump-outputs directory: under 64 MB with the .npy headers
+
+
+def step_outputs(bodies, man, joints, pairs, aabbs) -> dict:
+    """What a caller of one step receives: the bodies' new state, the contact impulses, the joint forces, the number of new pairs the
+    broad phase found and, when there are any, their columns, and its persistent order (the retained intervals only: the rest of
+    order_out is not written).  A steady-state snapshot has every current pair in its contact graph, so its count of new pairs is 0."""
+    out = {k: getattr(bodies, k) for k in ("position", "rotation", "linear_velocity", "angular_velocity")}
+    out.update({k: getattr(man, k) for k in ("warm_start_normal_impulse", "warm_start_tangent_impulse", "normal_impulse")})
+    for t, j in ({} if joints is None else joints.types).items():
+        for k in ("force", "torque"):
+            if getattr(j, k) is not None:
+                out[f"joint{int(t)}_{k}"] = getattr(j, k)
+    out["pair_count"] = np.array([pairs.count])
+    if pairs.count:
+        out.update({f"pairs_{k}": getattr(pairs, k)[:pairs.count] for k in ("collider1", "collider2", "body1", "body2", "flags")})
+    if aabbs.order_out is not None:
+        out["order"] = aabbs.order_out[:aabbs.retained_count]
+    return out
+
+
+def dump_outputs(out_dir: str, arrays: dict) -> None:
+    """<out_dir>/<name>.npy for every array: float columns in their own type, integer columns as float64 (exact below 2**53).  When the
+    arrays exceed DUMP_BUDGET, each keeps the same seeded sample of its rows (the same rows for arrays of the same length, at least one
+    row), so that the dumps of two builds still compare element for element.  An array without elements is not written."""
+    out = {k: np.array(v, dtype=v.dtype if v.dtype in (np.float32, np.float64) else np.float64) for k, v in arrays.items() if v.size}
+    total = sum(v.nbytes for v in out.values())
+    if total > DUMP_BUDGET:
+        share = DUMP_BUDGET / total
+        for k, v in out.items():
+            rows = np.random.default_rng(0).choice(v.shape[0], max(1, int(v.shape[0] * share)), replace=False)
+            out[k] = v[np.sort(rows)]
+    path = Path(out_dir)
+    path.mkdir(parents=True, exist_ok=True)
+    for k, v in out.items():
+        np.save(path / f"{k}.npy", v)
+
+
 def pin_columns(ctx, obj):
     """Move every numpy column of a Bodies/Manifolds/Aabbs dataclass into pinned host memory."""
     for k, v in list(obj.__dict__.items()):
@@ -209,6 +250,10 @@ def run_gpu(args, info):
     span_ms = timer.stop_ms()
     barrier()
     wall_resident = time.perf_counter() - t0
+    if args.dump_outputs and rank == 0:     # every run restarts from the uploaded snapshot: this is what the last timed step computed
+        ctx.broadphase_download(pairs_out)
+        ctx.solver_download()
+        dump_outputs(args.dump_outputs, step_outputs(bodies, man, joints, pairs_out, aabbs))
     # ---- the same loop with the per-call device times read back (stage breakdown, launch count); results are downloaded here
     mega_ms, bp_ms, launches, mode = 0.0, 0.0, 0, None
     n_break = min(K, 10)
@@ -592,14 +637,14 @@ def cpu_arm(args, prm, bodies, man, aabbs, sample_steps: int, joints=None, keep:
     threads = os.cpu_count() or 1
     t_total = 0.0
     for i in range(sample_steps):
-        b, m = bodies.copy(), man.copy()
+        b, m, j = bodies.copy(), man.copy(), None if joints is None else joints.copy()
         a = api.Aabbs(**{k: (v.copy() if isinstance(v, np.ndarray) else v) for k, v in aabbs.__dict__.items()})
         t0 = time.perf_counter()
         pairs = oracle_lib.broadphase(a, capacity=1 << 20)
-        oracle_lib.solver_step(prm, b, m, None if joints is None else joints.copy(), threads=threads)
+        oracle_lib.solver_step(prm, b, m, j, threads=threads)
         t_total += time.perf_counter() - t0
         if keep is not None and i == 0:
-            keep.update(bodies=b, manifolds=m, pairs=pairs, order=a.order_out)
+            keep.update(bodies=b, manifolds=m, joints=j, pairs=pairs, aabbs=a, order=a.order_out)
     return {"value": sample_steps / t_total, "unit": "steps/s", "cores": threads, "kind": "port",
             "sample": f"{sample_steps} full steps of the same snapshot (SAP single-threaded + solver stage colour-parallel on {threads} threads)",
             "ms_per_step": t_total / sample_steps * 1e3}
@@ -614,7 +659,10 @@ def run_reference(args, rank: int, world: int):
     prm.solver_iterations = args.solver_iterations
     if args.warmup:
         cpu_arm(args, prm, bodies, man, aabbs, args.warmup, joints)
-    cb = cpu_arm(args, prm, bodies, man, aabbs, args.steps, joints)
+    keep = {}
+    cb = cpu_arm(args, prm, bodies, man, aabbs, args.steps, joints, keep=keep)
+    if args.dump_outputs:     # every step starts from the same snapshot: the first step's outputs are the last step's
+        dump_outputs(args.dump_outputs, step_outputs(keep["bodies"], keep["manifolds"], keep["joints"], keep["pairs"], keep["aabbs"]))
     B, M, P = bodies.count, man.count, int(man.penetration.shape[0])
     sname = "f64" if bodies.position.dtype == np.float64 else "f32"
     cfg = workload_config(sc, prm, B, M, P, 0 if joints is None else joints.count, args.settle, sname, int(prm.solver_iterations))
@@ -641,11 +689,17 @@ def main():
     ap.add_argument("--no-partition", action="store_true", help="skip the one-scene-over-N-GPUs arms")
     ap.add_argument("--no-pass", action="store_true", help="skip the single solver-pass roofline measurement")
     ap.add_argument("--no-resident", action="store_true", help="e2e = round 1's host-manifold arm only")
-    ap.add_argument("--partition-steps", type=int, default=10)
+    ap.add_argument("--partition-steps", type=int, default=None, help="timed steps of the partition arms (default: --steps)")
     ap.add_argument("--partition-slab-scene", default="spheres1m", choices=sorted(SCENES))
     ap.add_argument("--partition-island-scene", default="ragdolls5k", choices=sorted(SCENES))
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the timed path computed in its last step as DIR/<name>.npy (float32/float64, at most 64 MB in all)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
+    if args.partition_steps is None:
+        args.partition_steps = args.steps
     if args.settle is None:
         args.settle = SCENES[args.scene][2]
     if args.scene != "stack100k":
